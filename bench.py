@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Headline benchmark: Taylor steps/s (fp64, batch) of outer_ss_long_term_batch on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+The benchmark writes nothing into the source tree: the helpers it compiles at run time (the generated CPU stepper, the
+C++ end-to-end tool) go to a temporary directory that is removed at exit.
 
 Workload (BASELINE.json configs[1]): the 6-body outer Solar System of benchmark/outer_ss_long_term_batch.cpp
 (model::nbody(6), masses/G/ICs of :60-94, high_accuracy = true, tol = eps -> order 20), 1,048,576 perturbed
@@ -21,21 +24,27 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree either
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "oracle")):
     if p not in sys.path:
         sys.path.insert(0, p)
 
+# Lanes of the fixed sample that --dump-outputs writes: 65,536 lanes x 44 float64 values (lane indices included) = 23 MB.
+DUMP_LANES = 1 << 16
+DUMP_SEED = 2024
+
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed leg (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=1 << 20, help="lanes per GPU")
@@ -50,7 +59,29 @@ def parse_args():
     ap.add_argument("--lanes-per-thread", type=int, default=0)
     ap.add_argument("--block-threads", type=int, default=0)
     ap.add_argument("--blocks-per-sm", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (final state, times, last step size, "
+                         "propagate results) for a fixed sample of %d lanes of rank 0 as float64 DIR/<name>.npy"
+                         % DUMP_LANES)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    return args
+
+
+_SCRATCH = None
+
+
+def scratch_dir():
+    """Private temporary directory for what the benchmark compiles at run time (removed at exit)."""
+    global _SCRATCH
+    if _SCRATCH is None:
+        _SCRATCH = tempfile.TemporaryDirectory(prefix="heyoka_b200_bench_")
+    return _SCRATCH.name
 
 
 def measured_peaks():
@@ -166,6 +197,7 @@ class CpuBaseline:
         import oracle
         from common import outer_ss_batch_state
         self.P, self.cores, self.oracle, self.codegen = P, cores, oracle, codegen
+        codegen.BUILD = scratch_dir()
         self.jets = {w: codegen.Jet(P, w) for w in (4, 8)}  # compiled outside of every timed region
         cal = outer_ss_batch_state(8 * cores, perturb=perturb, seed=7)
         self.rates = {}
@@ -252,19 +284,29 @@ def run_reference(args):
     }))
 
 
-def cpp_class_e2e(batch, tfinal, perturb):
+def dump_outputs(out_dir, n, dev, arrays):
+    """Writes the lanes of a fixed sample (DUMP_LANES lanes drawn with DUMP_SEED, ascending; all lanes if the batch is
+    smaller) of each device array [..., n] as float64 out_dir/<name>.npy, plus their indices as lanes.npy. The inputs
+    depend only on the arguments, so two builds run with the same arguments can be compared file by file."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    lanes = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_LANES), replace=False))
+    idx = torch.from_numpy(lanes).to(dev)
+    np.save(os.path.join(out_dir, "lanes.npy"), lanes.astype(np.float64))
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(t.dim() - 1, idx).double().cpu().numpy())
+
+
+def cpp_class_e2e(batch, steps, tfinal, perturb):
     """The same workload through the drop-in C++ class (tools/bench_cpp_e2e.cpp): host std::vector buffers in and out,
-    the call a heyoka user makes. One line per host_sync mode; None if the tool cannot be built."""
-    exe = os.path.join(ROOT, "build", "bench_cpp_e2e")
+    the call a heyoka user makes. One line per host_sync mode; an error record if the tool cannot be built."""
+    exe = os.path.join(scratch_dir(), "bench_cpp_e2e")
     src = os.path.join(ROOT, "tools", "bench_cpp_e2e.cpp")
     lib = os.path.join(ROOT, "heyoka_b200", "lib")
     try:
-        if not os.path.exists(exe) or os.path.getmtime(exe) < max(os.path.getmtime(src), os.path.getmtime(
-                os.path.join(lib, "libheyoka_b200.so"))):
-            os.makedirs(os.path.dirname(exe), exist_ok=True)
-            subprocess.run(["g++", "-std=c++17", "-O2", "-I" + os.path.join(ROOT, "include"), src, "-o", exe, "-L" + lib,
-                            "-lheyoka_b200", "-Wl,-rpath," + lib], check=True, capture_output=True)
-        res = subprocess.run([exe, str(batch), "2", repr(float(tfinal)), repr(float(perturb))], capture_output=True,
+        subprocess.run(["g++", "-std=c++17", "-O2", "-I" + os.path.join(ROOT, "include"), src, "-o", exe, "-L" + lib,
+                        "-lheyoka_b200", "-Wl,-rpath," + lib], check=True, capture_output=True)
+        res = subprocess.run([exe, str(batch), str(steps), repr(float(tfinal)), repr(float(perturb))], capture_output=True,
                              text=True, timeout=600, check=True)
         return [json.loads(line) for line in res.stdout.splitlines() if line.startswith("{")]
     except Exception as e:  # noqa: BLE001 - a reported extra, never fatal for the bench line
@@ -381,6 +423,11 @@ def main():
         assert bool(torch.equal(g[rank, :P.n_eq * n], t_state)), "the gathered block differs from the local state"
     launches = b.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # (Before the end-to-end leg below, which reuses the batch's buffers.)
+        dump_outputs(args.dump_outputs, n, dev, {
+            "state": t_state.view(P.n_eq, n), "time_hi": t_thi, "time_lo": t_tlo, "last_h": small[2],
+            "outcome": small[5].view(torch.int64), "min_h": small[3], "max_h": small[4], "n_steps": t_nsteps})
 
     # ---- end-to-end through the host-buffer API: pinned host -> device, propagate, device -> pinned host ----
     h_state = torch.from_numpy(st_host).pin_memory()
@@ -413,7 +460,7 @@ def main():
     e2e_step()
     sync_all()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n_e2e = max(2, min(args.steps, 3))
+    n_e2e = args.steps
     e0.record(stream)
     t_wall = time.perf_counter()
     for _ in range(n_e2e):
@@ -488,7 +535,7 @@ def main():
             "clocks": clocks,
         }
         if world == 1 and not args.no_cpp_e2e:
-            out["e2e_cpp_class"] = cpp_class_e2e(n, args.tfinal, args.perturb)
+            out["e2e_cpp_class"] = cpp_class_e2e(n, args.steps, args.tfinal, args.perturb)
         if not args.no_cpu_baseline and world == 1:
             cores = host_cores()
             cb = CpuBaseline(P, cores, args.perturb)

@@ -1159,6 +1159,8 @@ void hy_batch::ev_setup(std::uint32_t n_te_, const std::int32_t *dirs, const dou
     E.cd = keep(dalloc<double>(B * 2u * std::max(n_te, 1u)));
     E.cd_on = keep(dalloc<unsigned char>(B * std::max(n_te, 1u)));
     HY_CUDA_CHECK(cudaMemset(E.cd_on, 0, B * std::max(n_te, 1u)));
+    // (hy_batch_get_cooldowns() reports every lane, also those that have not been in a cooldown yet.)
+    HY_CUDA_CHECK(cudaMemset(E.cd, 0, sizeof(double) * B * 2u * std::max(n_te, 1u)));
     E.cand = keep(dalloc<std::uint32_t>(B * n_ev));
     E.counters = keep(dalloc<unsigned>(4));
     E.rec_cap = static_cast<std::uint32_t>(std::min<std::size_t>(std::max<std::size_t>(B * n_ev, 1024u), 1u << 26));

@@ -133,8 +133,10 @@ int main()
             // x(t) = x0 cos t + v0 sin t
             REQUIRE(std::abs(by_ptr[1] - (0.1 * std::cos(1.5) + 1.1 * std::sin(1.5))) < 1e-13);
             // get_times() / get_tcs() (include/heyoka/continuous_output.hpp:198-199): (n_steps + 2) rows of times (start,
-            // the end of every iteration, the padding), [n_steps][dim][order + 1][batch] Taylor coefficients; at the
-            // start of an iteration the output is the order-0 coefficients of that iteration.
+            // the end of every iteration, the padding), [n_steps][dim][order + 1][batch] Taylor coefficients. At the
+            // start of an iteration the output is the order-0 coefficients of that iteration: bit for bit at the
+            // starting time 0; elsewhere get_times() holds the high parts of double-length times, and the output at
+            // the high part is off by the low part lo (|lo| <= ulp(hi) / 2) times the order-1 coefficient, plus rounding.
             const auto n_steps = co->get_n_steps();
             const auto &tms = co->get_times();
             const auto &tcs = co->get_tcs();
@@ -143,11 +145,23 @@ int main()
             for (std::size_t i = 0; i < 4u; ++i) {
                 REQUIRE(tms[i] == 0. && tms[n_steps * 4u + i] == 5. && std::isinf(tms[(n_steps + 1u) * 4u + i]));
             }
+            const auto c_at = [&](std::size_t k, std::size_t var, std::size_t o, std::size_t i) {
+                return tcs[((k * 2u + var) * ord1 + o) * 4u + i];
+            };
             for (std::size_t k = 0; k < n_steps; ++k) {
                 const auto out = (*co)(tms.data() + k * 4u);
                 for (std::size_t var = 0; var < 2u; ++var) {
                     for (std::size_t i = 0; i < 4u; ++i) {
-                        REQUIRE(out[var * 4u + i] == tcs[((k * 2u + var) * ord1) * 4u + i]);
+                        double amp = 0.;
+                        for (std::size_t j = 0; j < n_steps; ++j) {
+                            amp = std::max(amp, std::abs(c_at(j, var, 0, i)));
+                        }
+                        const double t = std::abs(tms[k * 4u + i]);
+                        const double ulp = std::nextafter(t, std::numeric_limits<double>::infinity()) - t;
+                        const double tol = std::abs(c_at(k, var, 1, i)) * ulp
+                                           + 4. * std::numeric_limits<double>::epsilon() * amp;
+                        REQUIRE(std::abs(out[var * 4u + i] - c_at(k, var, 0, i)) <= tol);
+                        REQUIRE(k != 0u || out[var * 4u + i] == c_at(k, var, 0, i));
                     }
                 }
             }

@@ -14,13 +14,13 @@ from common import outer_ss_batch_state, sys_outer_ss, sys_tutorial
 
 pytestmark = pytest.mark.gpu
 
+N_DEVICES = hb.lib.hy_device_count()
+SEVERAL_GPUS = pytest.mark.skipif(N_DEVICES < 2, reason="needs two or more GPUs")
+
 
 def _device_lists():
-    n = hb.lib.hy_device_count()
-    lists = [[0, 0, 0]]  # three shards on one GPU: uneven blocks of lanes
-    if n > 1:
-        lists.append(list(range(n)))
-    return lists
+    # three shards on one GPU (uneven blocks of lanes); one shard per GPU of the machine
+    return [[0, 0, 0], pytest.param(list(range(max(N_DEVICES, 2))), marks=SEVERAL_GPUS)]
 
 
 def _same(a, b):
@@ -110,7 +110,7 @@ def test_sharded_with_parameters_and_time():
     # (propagate_grid() and continuous output of this sharded batch: tests/test_zz_gpu_late_additions.py)
 
 
-@pytest.mark.parametrize("devs", [None, [0, 0, 0]] + ([[0, 1]] if hb.lib.hy_device_count() >= 2 else []))
+@pytest.mark.parametrize("devs", [None, [0, 0, 0], pytest.param([0, 1], marks=SEVERAL_GPUS)])
 def test_propagate_until_host_one_call(devs):
     """hy_batch_propagate_until_host(): upload + propagate_until + downloads in one call, on one device, on one device in
     three pipelined sub-batches (the same device listed three times) and on two devices: bit-identical to the separate
