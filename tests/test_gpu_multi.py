@@ -6,6 +6,8 @@ reference's global exits of propagate_until() and its last_h semantics, which co
 
 The shards may live on the same GPU (device list [0, 0, 0]: what runs on a one-GPU box) or on every GPU of the box
 ("all")."""
+import re
+
 import numpy as np
 import pytest
 
@@ -19,8 +21,8 @@ SEVERAL_GPUS = pytest.mark.skipif(N_DEVICES < 2, reason="needs two or more GPUs"
 
 
 def _device_lists():
-    # three shards on one GPU (uneven blocks of lanes); one shard per GPU of the machine
-    return [[0, 0, 0], pytest.param(list(range(max(N_DEVICES, 2))), marks=SEVERAL_GPUS)]
+    # one shard; three shards on one GPU (uneven blocks of lanes); one shard per GPU of the machine
+    return [[0], [0, 0, 0], pytest.param(list(range(max(N_DEVICES, 2))), marks=SEVERAL_GPUS)]
 
 
 def _same(a, b):
@@ -110,7 +112,22 @@ def test_sharded_with_parameters_and_time():
     # (propagate_grid() and continuous output of this sharded batch: tests/test_zz_gpu_late_additions.py)
 
 
-@pytest.mark.parametrize("devs", [None, [0, 0, 0], pytest.param([0, 1], marks=SEVERAL_GPUS)])
+def test_single_shard_refuses_single_device_calls():
+    """A batch made by hy_batch_create_multi() with one device is one shard, and still refuses the entry points that
+    only a plain batch has."""
+    batch = 8
+    b = hb.Batch(hb.Program(sys_outer_ss()), batch, device=[0])
+    assert b.n_shards == 1
+    for exc, name, call in ((ValueError, "hy_batch_get_ptrs()", lambda: b.ptrs()),
+                            (ValueError, "hy_batch_set_stream()", lambda: b.set_stream(0)),
+                            (ValueError, "hy_batch_propagate_until_dev()", lambda: b.propagate_until_dev(0)),
+                            (NotImplementedError, "propagate_grid()", lambda: b.propagate_grid(np.zeros((1, batch)))),
+                            (NotImplementedError, "Continuous output", lambda: b.propagate_until_cout(np.ones(batch)))):
+        with pytest.raises(exc, match=re.escape(name + " is not available on a multi-device batch")):
+            call()
+
+
+@pytest.mark.parametrize("devs", [None, [0], [0, 0, 0], pytest.param([0, 1], marks=SEVERAL_GPUS)])
 def test_propagate_until_host_one_call(devs):
     """hy_batch_propagate_until_host(): upload + propagate_until + downloads in one call, on one device, on one device in
     three pipelined sub-batches (the same device listed three times) and on two devices: bit-identical to the separate
